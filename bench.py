@@ -15,9 +15,9 @@ resident in HBM, static camera (steady state).  Also on the line:
                    of the counters plus the visible command / cluster-index slabs (conservative: everything travels)
   e2e_incremental  what the reference's frame loop moves (niagara.cpp:1362-1411): CullData + the animated draws H2D
                    (scatter), counters D2H
-  moving_camera    a second timed region with the camera yawing every step, so that the late pass emits clusters and flips
-                   visibility bits (the compaction / atomics write path)
-  task_shading     the frame with meshlet.task.glsl's submission mode (nvc_taskcull) instead of the cluster passes
+  moving_camera    a second timed region of --steps frames with the camera yawing 0.2 degrees every step, so that the late pass
+                   emits clusters and flips visibility bits (the compaction / atomics write path)
+  task_shading     --steps frames with meshlet.task.glsl's submission mode (nvc_taskcull) instead of the cluster passes
   roofline         of whichever kernel dominates the step, with that pass's algorithmic bytes (SURVEY §8(d))
 The CPU arms (cpu_baseline, --impl reference) run oracle/ only; they never load the product library.
 """
@@ -54,7 +54,62 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-extras", action="store_true", help="skip the moving-camera and task-shading regions")
     ap.add_argument("--gather", default="mc", choices=["ce", "sm", "mc", "fused", "nccl", "none"], help="multi-GPU exchange of the late MeshTaskCommand slabs + counters: ce = copy-engine peer pushes over NVLink (no SMs), mc = one NVSwitch-multicast store kernel per rank (symmetric memory), fused = the late drawcull itself stores its commands through the multicast mapping, nccl = ncclAllGather, none = skip")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last step computed (per pass: counters, task commands and clusters in a canonical order; visibility bits, depth pyramid) as DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_ARRAY_BYTES = 12 << 20  # per dumped array, shared by the ranks: a larger one is written as a fixed, seeded sample of its rows (a dump stays under 64 MB)
+
+
+def pass_outputs(path):
+    """What the path's buffers hold after a cull + cluster pass: counters, the live task commands and the (drawId, meshlet)
+    pairs of the emitted clusters, both sorted — their order in the buffers depends on the scheduling of the device's atomics,
+    their content does not."""
+    import oracle_lib
+    import torch
+
+    torch.cuda.synchronize()
+    dccb, ccb = path.read_counts()
+    cmds = path.read_task_commands(int(dccb[1]) * 64)
+    return {
+        "dccb": dccb,
+        "ccb": ccb,
+        "commands": oracle_lib.sorted_commands(cmds[: min(int(dccb[0]), len(cmds))]),
+        "clusters": oracle_lib.cluster_pairs(path.read_cluster_indices(min(int(ccb[0]), path.cib.numel())), cmds),
+    }
+
+
+def frame_state(path):
+    """visibility state and depth pyramid at the end of a frame"""
+    return {"dvb": path.dvb.cpu().numpy().astype(np.uint32), "mvb": path.mvb.cpu().numpy().view(np.uint32), "pyramid": path.depthPyramid.cpu().numpy()}
+
+
+def dump_outputs(out_dir, passes, state, prefix="", array_bytes=DUMP_ARRAY_BYTES):
+    """Writes what a caller of the frame receives over one step, as float64 (integers, exact) or float32 (depth): per pass (column
+    0: 0 = early, 1 = late) the counters, task commands and clusters; the visibility bits and the pyramid at the end of the step."""
+
+    def rows(columns_of):
+        """one row per item of every pass: the pass, then the item's columns"""
+        return np.concatenate([np.stack([np.full(len(cols[0]), i, np.float64)] + [c.astype(np.float64) for c in cols], 1) for i, cols in enumerate(map(columns_of, passes))])
+
+    arrays = {
+        "draw_command_count": np.stack([p["dccb"] for p in passes]).astype(np.float64),
+        "cluster_count": np.stack([p["ccb"] for p in passes]).astype(np.float64),
+        "task_commands": rows(lambda p: [p["commands"][f] for f in p["commands"].dtype.names]),
+        "clusters": rows(lambda p: [p["clusters"] >> np.uint64(32), p["clusters"] & np.uint64(0xFFFFFFFF)]),
+        "draw_visibility": state["dvb"].astype(np.float64),
+        "meshlet_visibility": state["mvb"].astype(np.float64),
+        "depth_pyramid": state["pyramid"].astype(np.float32),
+    }
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        keep = array_bytes // max(1, a[:1].nbytes)
+        if len(a) > keep:
+            a = a[np.sort(np.random.default_rng(0).choice(len(a), keep, replace=False))]
+        np.save(os.path.join(out_dir, prefix + name + ".npy"), np.ascontiguousarray(a))
 
 
 def load_peaks():
@@ -549,8 +604,8 @@ def main():
     drain()
     torch.cuda.synchronize()
 
-    def probe(cull):
-        """one frame with the per-pass work counts read back (untimed)"""
+    def probe(cull, keep=None):
+        """one frame with the per-pass work counts read back (untimed); keep: a list that receives pass_outputs() of both passes"""
         reached = int((path.dvb != 0).sum().item())
         mvb_set_before = None
         path.dcb = dcb_early
@@ -561,6 +616,8 @@ def main():
         path.render_clusters(cull, late=False, cluster_backface=True)
         torch.cuda.synchronize()
         ccb_e = path.ccb.cpu().numpy().astype(np.uint32)
+        if keep is not None:
+            keep.append(pass_outputs(path))  # (the late pass overwrites cib)
         if produced is not None:
             depth.zero_()
             path.raster_depth(cull, produced["proj"], produced["vertices"], produced["meshletdata"], depth)
@@ -573,6 +630,8 @@ def main():
         path.render_clusters(cull, late=True, cluster_backface=True)
         torch.cuda.synchronize()
         ccb_l = path.ccb.cpu().numpy().astype(np.uint32)
+        if keep is not None:
+            keep.append(pass_outputs(path))
         if produced is not None:
             path.raster_depth(cull, produced["proj"], produced["vertices"], produced["meshletdata"], depth)
         return {
@@ -672,6 +731,22 @@ def main():
 
     # headline = graph replay when it ran (that is how a host would drive the frame), eager otherwise
     max_ms = graph_ms["median"] if graph_ms else min(eager_ms, plain_ms)
+    if args.dump_outputs:
+        # The early pass's commands and clusters of the last timed step are gone (the late pass reuses the buffers): the same frame
+        # runs once more, untimed, from the state the timed steps left, with both passes read back (without the multi-GPU exchange).
+        # The static camera is in a steady state, so it must reproduce the last timed step exactly — which also shows that leaving the
+        # exchange out did not change a rank's own outputs; every rank checks, and all of them agree before anything is written.
+        # Each rank writes its own outputs, with a share of the size limit.
+        last = dict(pass_outputs(path), **frame_state(path))
+        passes = []
+        probe(cd, passes)
+        again = dict(passes[1], **frame_state(path))
+        same = torch.tensor([int(all(np.array_equal(last[k], again[k]) for k in last))], dtype=torch.int32, device=dev)
+        if world > 1:
+            dist.all_reduce(same, op=dist.ReduceOp.MIN)
+        if not int(same.item()):
+            raise SystemExit("bench.py --dump-outputs: the replayed frame differs from the last timed step (no steady state)")
+        dump_outputs(args.dump_outputs, passes, again, "rank%d_" % rank if world > 1 else "", DUMP_ARRAY_BYTES // world)
 
     counts = torch.tensor([tested_per_step, draws_per_step], dtype=torch.float64, device=dev)
     if world > 1:
@@ -730,12 +805,11 @@ def main():
 
     def run_moving_camera():
         """yaw 0.2 degrees per step: the late pass now emits clusters and flips visibility bits"""
-        KM = max(10, min(60, K))
-        cams = [host.make_camera(orientation=host.quat_from_axis_angle((0.0, 1.0, 0.0), np.radians(0.2 * (k + 1)))) for k in range(KM)]
+        cams = [host.make_camera(orientation=host.quat_from_axis_angle((0.0, 1.0, 0.0), np.radians(0.2 * (k + 1)))) for k in range(K)]
         cds = [host.cull_data(c, scene.screen[0], scene.screen[1], D) for c in cams]
         dvb0, mvb0 = path.dvb.clone(), path.mvb.clone()
-        evm = new_events(KM)
-        mv_ms = timed(lambda k: frame(cds[k], evm[k]), KM)
+        evm = new_events(K)
+        mv_ms = timed(lambda k: frame(cds[k], evm[k]), K)
         mv_pass, _ = passes_of(evm)
         # replay the same camera path from the same state, untimed, reading the work counts of every step
         path.dvb.copy_(dvb0)
@@ -749,10 +823,10 @@ def main():
         late_ms = float(mv_pass[:, 4].mean())
         late_bytes = lm["tested_late"] * 24 + lm["cmds_late"] * 20 + lm["draws_late"] * 48 + 2 * lm["tested_late"] / 8.0 + 4 * lm["emitted_late"]
         return {
-            "what": "camera yaws 0.2 degrees per step (%d steps): draws enter / leave the frustum, occlusion changes, the late cluster pass emits clusters and rewrites visibility bits" % KM,
+            "what": "camera yaws 0.2 degrees per step (%d steps): draws enter / leave the frustum, occlusion changes, the late cluster pass emits clusters and rewrites visibility bits" % K,
             "value": float(t2.item()) / (mv_ms * 1e-3),
             "unit": "meshlets/s",
-            "ms_per_step": mv_ms / KM,
+            "ms_per_step": mv_ms / K,
             "passes_ms": {n: float(mv_pass[:, i].mean()) for i, n in enumerate(NAMES)},
             "per_step_mean": lm,
             "late_cluster_roofline": {"algorithmic_bytes_per_launch": late_bytes, "kernel_ms": late_ms, "achieved": late_bytes / (late_ms * 1e-3) / 1e9, "peak": peak_gbs, "frac": late_bytes / (late_ms * 1e-3) / 1e9 / peak_gbs, "unit": "GB/s"},
@@ -763,19 +837,18 @@ def main():
         ncmd_cap = (max(pr["cmds_early"], pr["cmds_late"]) + 63) // 64 * 64 + 64
         payloads = torch.zeros(ncmd_cap * 256, dtype=torch.uint8, device=dev)
         emit_counts = torch.zeros(ncmd_cap, dtype=torch.int32, device=dev)
-        KT = max(5, min(20, K))
         for _ in range(2):
             frame(cd, task=(payloads, emit_counts))
-        evt = new_events(KT)
-        t_ms = timed(lambda k: frame(cd, evt[k], task=(payloads, emit_counts)), KT)
+        evt = new_events(K)
+        t_ms = timed(lambda k: frame(cd, evt[k], task=(payloads, emit_counts)), K)
         t_pass, _ = passes_of(evt)
         tk_ms = float(t_pass[:, 4].mean())
         tk_bytes = pr["tested_late"] * 24 + pr["cmds_late"] * 20 + pr["draws_late"] * 48 + 2 * pr["tested_late"] / 8.0 + 4 * pr["emitted_late"] + 4 * pr["cmds_late"]
         return {
-            "what": "the frame with meshlet.task.glsl's submission mode: nvc_taskcull writes one 256-byte payload + emit count per task command instead of cib/ccb (%d steps)" % KT,
-            "value": tested_all * KT / (t_ms * 1e-3),
+            "what": "the frame with meshlet.task.glsl's submission mode: nvc_taskcull writes one 256-byte payload + emit count per task command instead of cib/ccb (%d steps)" % K,
+            "value": tested_all * K / (t_ms * 1e-3),
             "unit": "meshlets/s",
-            "ms_per_step": t_ms / KT,
+            "ms_per_step": t_ms / K,
             "passes_ms": {n.replace("clustercull", "taskcull"): float(t_pass[:, i].mean()) for i, n in enumerate(NAMES)},
             "late_taskcull_roofline": {"algorithmic_bytes_per_launch": tk_bytes, "kernel_ms": tk_ms, "achieved": tk_bytes / (tk_ms * 1e-3) / 1e9, "peak": peak_gbs, "frac": tk_bytes / (tk_ms * 1e-3) / 1e9 / peak_gbs, "unit": "GB/s"},
         }

@@ -23,3 +23,14 @@ extern "C" int cookhost_meshlet_bounds(const NvcVertex* vertices, uint32_t verte
 	}
 	return 0;
 }
+
+// the product's fp16 conversions (meshopt_quantizeHalf / meshopt_dequantizeHalf restated), for preparing test inputs
+extern "C" uint16_t cookhost_quantize_half(float v)
+{
+	return nvc::cook::quantize_half(v);
+}
+
+extern "C" float cookhost_dequantize_half(uint16_t h)
+{
+	return nvc::cook::dequantize_half(h);
+}

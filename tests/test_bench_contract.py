@@ -1,5 +1,5 @@
 """CPU-only: the reference arm of bench.py (`--impl reference`, the CPU restatement on the host cores) prints ONE JSON
-line with the contract's keys; ranks other than 0 print nothing and exit 0."""
+line with the contract's keys; ranks other than 0 print nothing and exit 0; the reference's shaders run outside the tests."""
 import json
 import os
 import subprocess
@@ -27,6 +27,34 @@ def test_reference_arm_json_contract():
     assert d["value"] > 0 and d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["cores"] >= 1
     assert d["e2e"]["h2d_bytes_per_step"] == 0 and d["e2e"]["d2h_bytes_per_step"] == 0 and d["e2e"]["value"] == d["value"]
     assert "workload" in d["config"]
+    # the reference's own shaders, timed by a child process where they are built (informational)
+    import refshader_lib
+
+    shaders = d["cpu_baseline"]["reference_shaders"]
+    assert (shaders["value"] > 0) if refshader_lib.available() else ("unavailable" in shaders), shaders
+
+
+def test_reference_shader_path_outside_a_pinned_test():
+    """bench.py drives RefShaderPath outside any test: with the reference's shaders it runs them (and agrees with the oracle);
+    without them it refuses, instead of standing in for them with nothing to hold the stand-in to."""
+    import numpy as np
+    import pytest
+
+    import oracle_lib
+    import refshader_lib
+    from niagara_b200 import scenes
+
+    s = scenes.instanced_scene(os.path.join(ROOT, "tests", "golden", "kitten.nvcg"), 256)
+    if not refshader_lib.available():
+        with pytest.raises(RuntimeError):
+            refshader_lib.RefShaderPath(s.meshes, s.meshlets, s.draws, *s.screen)
+        return
+    r = refshader_lib.RefShaderPath(s.meshes, s.meshlets, s.draws, *s.screen)
+    o = oracle_lib.OraclePath(s.meshes, s.meshlets, s.draws, *s.screen)
+    for p in (r, o):
+        p.set_visibility_bits(s.visibility_bits)
+        p.frame(s.cull_data(), s.depth, cluster_backface=True)
+    assert np.array_equal(r.dccb, o.dccb) and np.array_equal(r.ccb, o.ccb) and np.array_equal(r.mvb, o.mvb)
 
 
 def test_reference_arm_other_ranks_are_silent():

@@ -56,18 +56,51 @@ def test_host_instantiation_reproduces_reference_cooker_animated():
     assert len(np.unique(want["cone_cutoff"])) > 3 and (want["radius"] != 0).all()
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="needs the reference checkout to cook kitten.obj / pirate.obj now")
+def _pirate_fixtures():
+    import importlib.util
+
+    spec = importlib.util.spec_from_file_location("make_pirate_fixtures", os.path.join(GOLDEN, "make_pirate_fixtures.py"))
+    mod = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(mod)
+    return mod
+
+
 def test_host_instantiation_reproduces_reference_cooker_real_meshes(tmp_path):
-    """792 + ~150 meshlets cooked by the reference right now (all LODs, short and long reference lists, wide cones)."""
+    """792 + ~300 meshlets cooked by the reference (all LODs, short and long reference lists, wide cones): right now where the
+    reference is present — the stored copies must then be what it writes — from kitten_cook.npz + kitten.nvcg, pirate_cook.npz
+    and pirate_glb.z.cache elsewhere (tests/golden/make_pirate_fixtures.py)."""
+    from refshader_lib import REFERENCE
+
+    fixtures = _pirate_fixtures()
     lib = _host_lib()
-    subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref"], check=True)
-    tool = os.path.join(ROOT, "oracle", "_ref", "write_cache")
+    live = os.path.isdir(os.path.join(REFERENCE, "src"))
+    if live:
+        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref", "REF=" + REFERENCE], check=True)
     total = 0
-    for name, src in (("kitten", "/root/reference/data/kitten.obj"), ("pirate", "/root/reference/extern/meshoptimizer/demo/pirate.obj"), ("pirateglb", "/root/reference/extern/meshoptimizer/demo/pirate.glb")):
-        subprocess.run([tool, str(tmp_path / name), src], check=True, stdout=subprocess.DEVNULL)
-        vertices, data, want = _inputs(str(tmp_path / (name + ".raw.cache")))
+    for name in ("kitten", "pirate", "pirate_glb"):
+        if live:
+            if name == "kitten":
+                subprocess.run([os.path.join(ROOT, "oracle", "_ref", "write_cache"), str(tmp_path / name), os.path.join(REFERENCE, "data", "kitten.obj")], check=True, stdout=subprocess.DEVNULL)
+            else:
+                fixtures.write_cache(str(tmp_path), name)
+            positions, data, want = fixtures.cook_inputs(str(tmp_path / (name + ".raw.cache")))
+            if name == "pirate":
+                stored = np.load(os.path.join(GOLDEN, "pirate_cook.npz"))
+                assert all(np.array_equal(stored[k], v) for k, v in (("positions", positions), ("meshletdata", data), ("meshlets", want)))
+            elif name == "pirate_glb":
+                assert open(tmp_path / "pirate_glb.z.cache", "rb").read() == open(os.path.join(GOLDEN, "pirate_glb.z.cache"), "rb").read()
+        elif name == "kitten":
+            z = np.load(os.path.join(GOLDEN, "kitten_cook.npz"))
+            positions, data, want = z["positions"], z["meshletdata"], layout.load_nvcg(os.path.join(GOLDEN, "kitten.nvcg"))[1]
+        elif name == "pirate":
+            z = np.load(os.path.join(GOLDEN, "pirate_cook.npz"))
+            positions, data, want = z["positions"], z["meshletdata"], z["meshlets"]
+        else:  # the reference's compressed cache, read by the product's decoders (checked against the reference's in test_scene_cache.py)
+            positions, data, want = fixtures.cook_inputs(os.path.join(GOLDEN, "pirate_glb.z.cache"))
+        vertices = np.zeros((len(positions), 8), dtype=np.uint16)
+        vertices[:, :3] = positions
         got = _scrub(want)
-        lib.cookhost_meshlet_bounds(vertices.ctypes.data, len(vertices) // 16, data.ctypes.data, len(data), got.ctypes.data, len(got))
+        lib.cookhost_meshlet_bounds(vertices.ctypes.data, len(vertices), data.ctypes.data, len(data), got.ctypes.data, len(got))
         _check(got, want, name)
         total += len(want)
     assert total > 900
@@ -131,13 +164,26 @@ def test_gpu_kernel_reproduces_reference_cooker():
         lib.nvc_destroy(ctx)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src") and not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libmeshopt_ref.so")), reason="needs the reference's meshoptimizer (oracle/_ref/libmeshopt_ref.so)")
-def test_host_instantiation_against_reference_bounds_on_random_meshlets():
+def test_host_instantiation_against_reference_bounds_on_random_meshlets(request):
     """Property test: random meshlets (smooth patches, random soups -> cones wider than a hemisphere, fans, degenerate and
     duplicated triangles, single triangles, collinear points) through meshopt_computeMeshletBounds + meshopt_quantizeHalf of
-    the reference's vendored library vs the product's nvc_cook.cuh: identical center / radius / cone bytes."""
-    if os.path.isdir("/root/reference/src"):
-        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref"], check=True)
+    the reference's vendored library vs the product's nvc_cook.cuh: identical center / radius / cone bytes.  Without the
+    reference library the inputs are quantised by the product's restatement of meshopt_quantizeHalf, and inputs and bounds
+    are held to the reference's, pinned per 100 cases."""
+    import reference_pins
+    import test_meshopt_decoders
+
+    live = test_meshopt_decoders.load_ref() is not None
+    with reference_pins.pinned(request, live):
+        _random_meshlet_bounds(live)
+
+
+def _random_meshlet_bounds(live):
+    lib = _host_lib()
+    lib.cookhost_quantize_half.restype = ctypes.c_ushort
+    lib.cookhost_quantize_half.argtypes = [ctypes.c_float]
+    if not live:
+        return _random_meshlet_cases(lib, None)
     mo = ctypes.CDLL(os.path.join(ROOT, "oracle", "_ref", "libmeshopt_ref.so"))
 
     class Bounds(ctypes.Structure):
@@ -150,8 +196,16 @@ def test_host_instantiation_against_reference_bounds_on_random_meshlets():
     mo.meshopt_quantizeHalf.argtypes = [ctypes.c_float]
     mo.meshopt_dequantizeHalf.restype = ctypes.c_float
     mo.meshopt_dequantizeHalf.argtypes = [ctypes.c_ushort]
-    lib = _host_lib()
+    return _random_meshlet_cases(lib, mo)
+
+
+def _random_meshlet_cases(lib, mo):
+    """mo: the reference's meshoptimizer, or None (the reference's results are then the pinned ones)"""
+    import reference_pins
+
+    quantize = lib.cookhost_quantize_half if mo is None else mo.meshopt_quantizeHalf
     rng = np.random.default_rng(77)
+    halves, bounds = [], []
     seen = {"degenerate": 0, "wide": 0, "cone": 0}
     for case in range(1500):
         vc = int(rng.integers(3, 65))
@@ -186,7 +240,9 @@ def test_host_instantiation_against_reference_bounds_on_random_meshlets():
             pos = np.stack([np.cos(a), np.sin(a), np.zeros(vc)], 1) * rng.uniform(0.5, 3) + rng.standard_normal((1, 3))
         else:  # tiny and huge coordinates (fp16 flush-to-zero / large magnitudes)
             pos = rng.standard_normal((vc, 3)) * (1e-5 if rng.random() < 0.5 else 2e4)
-        half = np.array([mo.meshopt_quantizeHalf(float(x)) for x in pos.reshape(-1)], np.uint16).reshape(vc, 3)
+        half = np.array([quantize(float(x)) for x in pos.reshape(-1)], np.uint16).reshape(vc, 3)
+        if mo is not None:
+            assert np.array_equal(half.reshape(-1), [lib.cookhost_quantize_half(float(x)) for x in pos.reshape(-1)]), case
         if grid is not None:
             tris = grid.copy()
         elif style == 4:
@@ -203,14 +259,15 @@ def test_host_instantiation_against_reference_bounds_on_random_meshlets():
         refs = np.arange(used, dtype=np.uint32) if rng.random() < 0.5 else rng.permutation(vc).astype(np.uint32)[:used]
         short = bool(rng.integers(0, 2))
 
-        # the reference: float positions = dequantised halves, indexed by (baseVertex-relative) reference
-        fpos = np.array([mo.meshopt_dequantizeHalf(int(h)) for h in half.reshape(-1)], np.float32).reshape(vc, 3)
-        b = mo.meshopt_computeMeshletBounds(refs.ctypes.data, tris.ctypes.data, tc, fpos.ctypes.data, vc, 12)
-        want = np.zeros(1, layout.MESHLET_DTYPE)
-        want["center"] = [mo.meshopt_quantizeHalf(b.center[k]) for k in range(3)]
-        want["radius"] = mo.meshopt_quantizeHalf(b.radius)
-        want["cone_axis"] = [b.cone_axis_s8[k] for k in range(3)]
-        want["cone_cutoff"] = b.cone_cutoff_s8
+        if mo is not None:
+            # the reference: float positions = dequantised halves, indexed by (baseVertex-relative) reference
+            fpos = np.array([mo.meshopt_dequantizeHalf(int(h)) for h in half.reshape(-1)], np.float32).reshape(vc, 3)
+            b = mo.meshopt_computeMeshletBounds(refs.ctypes.data, tris.ctypes.data, tc, fpos.ctypes.data, vc, 12)
+            want = np.zeros(1, layout.MESHLET_DTYPE)
+            want["center"] = [mo.meshopt_quantizeHalf(b.center[k]) for k in range(3)]
+            want["radius"] = mo.meshopt_quantizeHalf(b.radius)
+            want["cone_axis"] = [b.cone_axis_s8[k] for k in range(3)]
+            want["cone_cutoff"] = b.cone_cutoff_s8
 
         # the product: Vertex[] with the fp16 positions at baseVertex, meshletdata = references (+ pad) + triangle bytes
         vertices = np.zeros((base + vc, 8), np.uint16)
@@ -228,7 +285,14 @@ def test_host_instantiation_against_reference_bounds_on_random_meshlets():
         got = m.copy()
         got.view(np.uint8).reshape(1, 24)[:, :CULL_FIELDS] = 0xCD
         lib.cookhost_meshlet_bounds(vertices.ctypes.data, len(vertices), data.ctypes.data, len(data), got.ctypes.data, 1)
-        for f in ("center", "radius", "cone_axis", "cone_cutoff"):
-            assert np.array_equal(got[f], want[f]), (case, style, f, got[f], want[f])
-        seen["degenerate" if (b.radius == 0 and b.cone_cutoff_s8 == 0) else ("wide" if b.cone_cutoff_s8 == 127 and not any(b.cone_axis_s8) else "cone")] += 1
-    assert seen["degenerate"] > 50 and seen["wide"] > 200 and seen["cone"] > 300, seen
+        if mo is not None:
+            for f in ("center", "radius", "cone_axis", "cone_cutoff"):
+                assert np.array_equal(got[f], want[f]), (case, style, f, got[f], want[f])
+            seen["degenerate" if (b.radius == 0 and b.cone_cutoff_s8 == 0) else ("wide" if b.cone_cutoff_s8 == 127 and not any(b.cone_axis_s8) else "cone")] += 1
+        halves.append(half.reshape(-1))
+        bounds.append((want if mo is not None else got).view(np.uint8)[:CULL_FIELDS])
+        if len(bounds) == 100:
+            reference_pins.check("cases %d-%d: inputs, bounds" % (case - 99, case), np.concatenate(halves), np.concatenate(bounds))
+            halves, bounds = [], []
+    if mo is not None:  # (the pinned inputs are the reference's, so is their spread over the three kinds)
+        assert seen["degenerate"] > 50 and seen["wide"] > 200 and seen["cone"] > 300, seen

@@ -15,6 +15,7 @@ import pytest
 
 import emu_lib
 import oracle_lib
+import reference_pins
 import refshader_lib
 from niagara_b200 import host, layout, scenes
 
@@ -26,7 +27,13 @@ def _culler(name):
     PRODUCT's CUDA kernels under the CPU SIMT emulation (tests/cuda_emu)"""
     return {"oracle": oracle_lib.OraclePath, "reference-shaders": refshader_lib.RefShaderPath, "cuda-kernels-emulated": emu_lib.EmuPath}[name]
 
-pytestmark = pytest.mark.skipif(not refshader_lib.available(), reason="needs /root/reference or a prebuilt oracle/_ref/librefshader.so")
+
+
+@pytest.fixture(autouse=True)
+def _reference_pins(request):
+    """where the reference's shaders cannot run, its passes, mesh and vertex stages are stood in for and held to its pinned outputs"""
+    with reference_pins.pinned(request, refshader_lib.available()):
+        yield
 
 
 def _kitten_scene(golden_dir, n, screen):

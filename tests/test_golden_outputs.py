@@ -31,22 +31,21 @@ def test_oracle_reproduces_committed_vectors():
         assert a.tobytes() == b.tobytes(), k
 
 
-def test_reference_shaders_reproduce_committed_vectors():
+def test_reference_shaders_reproduce_committed_vectors(request):
     """The same scenarios executed by the reference's own GLSL (oracle/refshader, one host thread = in-order dispatch):
     every committed array, including the ORDER of the commands, comes out byte for byte."""
-    import pytest
-
+    import reference_pins
     import refshader_lib
 
-    if not refshader_lib.available():
-        pytest.skip("needs /root/reference or a prebuilt oracle/_ref/librefshader.so")
     want = np.load(os.path.join(ROOT, "tests", "golden", "c1_kitten_expected.npz"))
-    got = _maker().compute(refshader_lib.RefShaderPath)
-    for k in want.files:
-        if k == "a_lod":
-            continue  # a diagnostic output of the oracle only (the shaders do not export the selected LOD)
-        a, b = np.asarray(want[k]), np.asarray(got[k])
-        assert a.shape == b.shape and a.dtype == b.dtype and a.tobytes() == b.tobytes(), k
+    with reference_pins.pinned(request, refshader_lib.available()):
+        got = _maker().compute(refshader_lib.RefShaderPath)
+        for k in want.files:
+            if k == "a_lod":
+                continue  # a diagnostic output of the oracle only (the shaders do not export the selected LOD)
+            a, b = np.asarray(want[k]), np.asarray(got[k])
+            assert a.shape == b.shape and a.dtype == b.dtype and a.tobytes() == b.tobytes(), k
+            reference_pins.check(k, b)  # as the shaders wrote it, order included
 
 
 def test_config0_frustum_only_matches_numpy_restatement():

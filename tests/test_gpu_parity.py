@@ -135,21 +135,21 @@ def test_cuda_reproduces_committed_vectors(golden_dir):
     assert crc(pyr.view(np.uint32)) == want["b_pyramid_crc"]
 
 
-def test_cuda_vs_reference_shaders(golden_dir):
+def test_cuda_vs_reference_shaders(golden_dir, request):
     """The CUDA path against the reference's OWN GLSL shaders run on the host (oracle/_ref/librefshader.so: the text of
-    src/shaders/*.glsl compiled through oracle/refshader/glsl_shim.h by build(); the prebuilt library travels to the
-    GPU box).  Same bar as against the oracle: bit-exact, order inside dcb / cib aside."""
+    src/shaders/*.glsl compiled through oracle/refshader/glsl_shim.h).  Same bar as against the oracle: bit-exact, order
+    inside dcb / cib aside.  Without the library the oracle runs in its place, held to the reference's pinned outputs."""
+    import reference_pins
     import refshader_lib
 
-    if not refshader_lib.available():
-        pytest.skip("oracle/_ref/librefshader.so was not built (needs /root/reference at build time)")
-    s = scenes.instanced_scene(os.path.join(golden_dir, "kitten_pirate.nvcg"), 20000, screen=(1280, 720))
-    g, r = _run_frames(s, frames=2, checker=refshader_lib.RefShaderPath)
-    assert r.read_counts()[0][0] > 0
-    s = scenes.config2_scene(draw_count=50000, num_meshes=256, screen=(1024, 1024))
-    _run_frames(s, frames=2, checker=refshader_lib.RefShaderPath)
-    s = scenes.instanced_scene(os.path.join(golden_dir, "kitten.nvcg"), 3000)
-    _run_frames(s, frames=2, checker=refshader_lib.RefShaderPath, toggles=dict(mesh_shading=False, cluster_occlusion=False), mesh_shading=False)
+    with reference_pins.pinned(request, refshader_lib.available()):
+        s = scenes.instanced_scene(os.path.join(golden_dir, "kitten_pirate.nvcg"), 20000, screen=(1280, 720))
+        g, r = _run_frames(s, frames=2, checker=refshader_lib.RefShaderPath)
+        assert r.read_counts()[0][0] > 0
+        s = scenes.config2_scene(draw_count=50000, num_meshes=256, screen=(1024, 1024))
+        _run_frames(s, frames=2, checker=refshader_lib.RefShaderPath)
+        s = scenes.instanced_scene(os.path.join(golden_dir, "kitten.nvcg"), 3000)
+        _run_frames(s, frames=2, checker=refshader_lib.RefShaderPath, toggles=dict(mesh_shading=False, cluster_occlusion=False), mesh_shading=False)
 
 
 def test_scene_cache_and_animated_draws(golden_dir):
@@ -517,14 +517,21 @@ def test_c3_bistro_standin_two_pass(golden_dir):
     assert int(o.read_counts()[1][0]) >= 0 and len(early) + len(late) > 10000
 
 
-def test_two_phase_on_device_produced_depth(golden_dir):
+def test_two_phase_on_device_produced_depth(golden_dir, request):
     """The whole loop on the device with NO synthetic depth: early cull -> nvc_raster_depth -> pyramid of that depth -> late cull ->
     nvc_raster_depth, over a moving camera — against the oracle culling + the reference's mesh shader + the sequential test
-    rasteriser (oracle/refshader) doing the same on the CPU.  Depth images, cluster sets and visibility state must be identical."""
+    rasteriser (oracle/refshader) doing the same on the CPU.  Depth images, cluster sets and visibility state must be identical.
+    Without the reference's shaders their mesh stage is stood in for and held to its pinned outputs."""
+    import reference_pins
     import refshader_lib
 
-    if not refshader_lib.available():
-        pytest.skip("needs a prebuilt oracle/_ref/librefshader.so")
+    with reference_pins.pinned(request, refshader_lib.available()):
+        _two_phase_on_device_produced_depth(golden_dir)
+
+
+def _two_phase_on_device_produced_depth(golden_dir):
+    import refshader_lib
+
     torch = _torch()
     from test_end_to_end_raster import _kitten_scene
 

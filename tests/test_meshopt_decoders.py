@@ -2,7 +2,11 @@
 _meshlet_stream, csrc/nvc_meshopt_decode.cpp + nvc_scene_cache.cpp) against the REFERENCE's vendored codec library
 (oracle/_ref/libmeshopt_ref.so: extern/meshoptimizer/src/{vertex,index,meshlet}codec.cpp compiled where they lie):
 random and structured inputs are encoded by the reference's encoders (both codec versions, all compression levels)
-and decoded by both sides; results must be identical, byte for byte."""
+and decoded by both sides; results must be identical, byte for byte.
+
+Without the reference library the decoders run on a fixed sample of the same cases: the streams the reference's encoders
+wrote for them (tests/golden/meshopt_streams.npz, made by tests/golden/make_meshopt_streams.py) and the reference decoder's
+outputs, pinned by reference_pins."""
 import ctypes
 import os
 import subprocess
@@ -10,20 +14,23 @@ import subprocess
 import numpy as np
 import pytest
 
+import reference_pins
 from niagara_b200.lib import load_library
+from refshader_lib import REFERENCE
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 REF_SO = os.path.join(ROOT, "oracle", "_ref", "libmeshopt_ref.so")
-
-pytestmark = pytest.mark.skipif(not (os.path.exists(REF_SO) or os.path.isdir("/root/reference/src")), reason="needs the reference's codecs (oracle/_ref/libmeshopt_ref.so)")
+STREAMS = os.path.join(ROOT, "tests", "golden", "meshopt_streams.npz")
 
 vp, sz = ctypes.c_void_p, ctypes.c_size_t
 
 
-@pytest.fixture(scope="module")
-def ref():
-    if os.path.isdir("/root/reference/src"):
-        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref"], check=True)
+def load_ref():
+    """The reference's codec library, or None where it is neither built nor buildable."""
+    if os.path.isdir(os.path.join(REFERENCE, "src")):
+        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref", "REF=" + REFERENCE], check=True)
+    if not os.path.exists(REF_SO):
+        return None
     lib = ctypes.CDLL(REF_SO)
     lib.meshopt_encodeVertexBufferBound.restype = sz
     lib.meshopt_encodeVertexBufferBound.argtypes = [sz, sz]
@@ -45,6 +52,35 @@ def ref():
     lib.meshopt_decodeMeshlet.restype = ctypes.c_int
     lib.meshopt_decodeMeshlet.argtypes = [vp, sz, sz, vp, sz, sz, vp, sz]
     return lib
+
+
+@pytest.fixture(scope="module")
+def ref():
+    return load_ref()
+
+
+@pytest.fixture(scope="module")
+def stored():
+    z = np.load(STREAMS)
+    ends = np.cumsum(z["sizes"].astype(np.int64))
+    return {str(k): z["streams"][e - n : e] for k, n, e in zip(z["keys"], z["sizes"], ends)}
+
+
+@pytest.fixture(autouse=True)
+def _reference_pins(request, ref):
+    with reference_pins.pinned(request, ref is not None):
+        yield
+
+
+def _stream(ref, stored, key, encode):
+    """The reference's stream for case `key`: encoded now (and equal to the stored copy, if any), or the stored copy;
+    None when the reference is absent and the case is not in the stored sample."""
+    if ref is None:
+        return stored.get(key)
+    stream = encode()
+    if key in stored:
+        assert np.array_equal(stored[key], stream), key
+    return stream
 
 
 def _p(a):
@@ -70,11 +106,9 @@ def _vertex_data(rng, count, stride, kind):
     raise ValueError(kind)
 
 
-@pytest.mark.parametrize("version", [0, 1])
-def test_vertex_codec_against_reference(ref, version):
-    ours = load_library()
+def vertex_cases(version):
+    """(key, data, level) of every vertex codec case, in the order the random inputs are drawn"""
     rng = np.random.default_rng(100 + version)
-    cases = 0
     for stride in (4, 8, 12, 16, 20, 32, 48, 64, 256):
         for count in (1, 2, 15, 16, 17, 255, 256, 257, 1000, 3000):
             for kind in ("random", "zeros", "smooth16", "floats", "sparse"):
@@ -82,21 +116,39 @@ def test_vertex_codec_against_reference(ref, version):
                     continue
                 data = np.ascontiguousarray(_vertex_data(rng, count, stride, kind))
                 for level in ((0, 1, 2, 3) if version == 1 else (2,)):
-                    buf = np.zeros(ref.meshopt_encodeVertexBufferBound(count, stride), np.uint8)
-                    n = ref.meshopt_encodeVertexBufferLevel(_p(buf), len(buf), _p(data), count, stride, level, version)
-                    assert n > 0
-                    stream = np.ascontiguousarray(buf[:n])
-                    want = np.zeros_like(data)
-                    assert ref.meshopt_decodeVertexBuffer(_p(want), count, stride, _p(stream), n) == 0
-                    assert np.array_equal(want, data)  # the codec is lossless
-                    got = np.full((count + 1, stride), 0xEE, np.uint8)
-                    assert ours.nvc_decode_vertex_stream(_p(got), count, stride, _p(stream), n) == 0, (stride, count, kind, level)
-                    assert np.array_equal(got[:count], data), (stride, count, kind, level)
-                    assert (got[count] == 0xEE).all()
-                    # a truncated or extended stream is rejected by both
-                    assert ours.nvc_decode_vertex_stream(_p(got), count, stride, _p(stream), n - 1) != 0
-                    cases += 1
-    assert cases > 400
+                    yield "vertex_v%d_%d_%d_%s_%d" % (version, stride, count, kind, level), data, level
+
+
+def encode_vertex(ref, data, level, version):
+    count, stride = data.shape
+    buf = np.zeros(ref.meshopt_encodeVertexBufferBound(count, stride), np.uint8)
+    n = ref.meshopt_encodeVertexBufferLevel(_p(buf), len(buf), _p(data), count, stride, level, version)
+    assert n > 0
+    stream = np.ascontiguousarray(buf[:n])
+    want = np.zeros_like(data)
+    assert ref.meshopt_decodeVertexBuffer(_p(want), count, stride, _p(stream), n) == 0
+    assert np.array_equal(want, data)  # the codec is lossless
+    return stream
+
+
+@pytest.mark.parametrize("version", [0, 1])
+def test_vertex_codec_against_reference(ref, stored, version):
+    ours = load_library()
+    cases = 0
+    for key, data, level in vertex_cases(version):
+        count, stride = data.shape
+        stream = _stream(ref, stored, key, lambda: encode_vertex(ref, data, level, version))
+        if stream is None:
+            continue
+        n = len(stream)
+        got = np.full((count + 1, stride), 0xEE, np.uint8)
+        assert ours.nvc_decode_vertex_stream(_p(got), count, stride, _p(stream), n) == 0, key
+        assert np.array_equal(got[:count], data), key
+        assert (got[count] == 0xEE).all()
+        # a truncated or extended stream is rejected by both
+        assert ours.nvc_decode_vertex_stream(_p(got), count, stride, _p(stream), n - 1) != 0
+        cases += 1
+    assert cases > (400 if ref is not None else 40)
 
 
 def _index_data(rng, triangles, kind):
@@ -117,42 +169,54 @@ def _index_data(rng, triangles, kind):
     raise ValueError(kind)
 
 
-@pytest.mark.parametrize("version", [0, 1])
-def test_index_codec_against_reference(ref, version):
-    ours = load_library()
+def index_cases(version):
     rng = np.random.default_rng(200 + version)
+    for triangles in (1, 2, 3, 16, 17, 100, 1000, 5000):
+        for kind in ("random", "strip", "grid", "jumps"):
+            yield "index_v%d_%d_%s" % (version, triangles, kind), np.ascontiguousarray(_index_data(rng, triangles, kind), dtype=np.uint32)
+
+
+def encode_index(ref, idx, version):
     ref.meshopt_encodeIndexVersion(version)
-    cases = 0
     try:
-        for triangles in (1, 2, 3, 16, 17, 100, 1000, 5000):
-            for kind in ("random", "strip", "grid", "jumps"):
-                idx = np.ascontiguousarray(_index_data(rng, triangles, kind), dtype=np.uint32)
-                buf = np.zeros(ref.meshopt_encodeIndexBufferBound(len(idx), 0xFFFFFFFF), np.uint8)
-                n = ref.meshopt_encodeIndexBuffer(_p(buf), len(buf), _p(idx), len(idx))
-                assert n > 0
-                stream = np.ascontiguousarray(buf[:n])
-                assert stream[0] == (0xE0 | version)
-                want = np.zeros_like(idx)
-                assert ref.meshopt_decodeIndexBuffer(_p(want), len(idx), 4, _p(stream), n) == 0
-                got = np.full(len(idx) + 3, 0xEEEEEEEE, np.uint32)
-                assert ours.nvc_decode_index_stream(_p(got), len(idx), _p(stream), n) == 0, (triangles, kind)
-                assert np.array_equal(got[: len(idx)], want), (triangles, kind)
-                assert (got[len(idx) :] == 0xEEEEEEEE).all()
-                # same triangles as the input, corners possibly rotated
-                a, b = idx.reshape(-1, 3), want.reshape(-1, 3)
-                assert ((a == b).all(1) | (np.roll(a, 1, 1) == b).all(1) | (np.roll(a, 2, 1) == b).all(1)).all()
-                assert ours.nvc_decode_index_stream(_p(got), len(idx), _p(stream), n - 1) != 0
-                cases += 1
+        buf = np.zeros(ref.meshopt_encodeIndexBufferBound(len(idx), 0xFFFFFFFF), np.uint8)
+        n = ref.meshopt_encodeIndexBuffer(_p(buf), len(buf), _p(idx), len(idx))
     finally:
         ref.meshopt_encodeIndexVersion(1)
-    assert cases == 32
+    assert n > 0
+    return np.ascontiguousarray(buf[:n])
 
 
-def test_meshlet_codec_against_reference(ref):
+@pytest.mark.parametrize("version", [0, 1])
+def test_index_codec_against_reference(ref, stored, version):
     ours = load_library()
-    rng = np.random.default_rng(300)
     cases = 0
-    for _ in range(600):
+    for key, idx in index_cases(version):
+        stream = _stream(ref, stored, key, lambda: encode_index(ref, idx, version))
+        if stream is None:
+            continue
+        n = len(stream)
+        assert stream[0] == (0xE0 | version)
+        got = np.full(len(idx) + 3, 0xEEEEEEEE, np.uint32)
+        assert ours.nvc_decode_index_stream(_p(got), len(idx), _p(stream), n) == 0, key
+        if ref is not None:
+            want = np.zeros_like(idx)
+            assert ref.meshopt_decodeIndexBuffer(_p(want), len(idx), 4, _p(stream), n) == 0
+            assert np.array_equal(got[: len(idx)], want), key
+        if key in stored:
+            reference_pins.check(key, want if ref is not None else got[: len(idx)])
+        assert (got[len(idx) :] == 0xEEEEEEEE).all()
+        # same triangles as the input, corners possibly rotated
+        a, b = idx.reshape(-1, 3), got[: len(idx)].reshape(-1, 3)
+        assert ((a == b).all(1) | (np.roll(a, 1, 1) == b).all(1) | (np.roll(a, 2, 1) == b).all(1)).all()
+        assert ours.nvc_decode_index_stream(_p(got), len(idx), _p(stream), n - 1) != 0
+        cases += 1
+    assert cases == (32 if ref is not None else len([k for k in stored if k.startswith("index_v%d_" % version)]))
+
+
+def meshlet_cases():
+    rng = np.random.default_rng(300)
+    for case in range(600):
         vc = int(rng.integers(3, 257)) if rng.random() < 0.3 else int(rng.integers(3, 65))
         tc = int(rng.integers(1, 257)) if rng.random() < 0.3 else int(rng.integers(1, 97))
         style = rng.integers(0, 4)
@@ -170,24 +234,42 @@ def test_meshlet_codec_against_reference(ref):
         else:  # large deltas: 3- and 4-byte groups
             refs = (rng.integers(0, 1 << 24, vc) * rng.integers(1, 200, vc)).astype(np.uint32)
             tris = rng.integers(0, vc, (tc, 3)).astype(np.uint8)
-        refs, tris = np.ascontiguousarray(refs), np.ascontiguousarray(tris)
-        buf = np.zeros(ref.meshopt_encodeMeshletBound(256, 256), np.uint8)
-        n = ref.meshopt_encodeMeshlet(_p(buf), len(buf), _p(refs), vc, _p(tris), tc)
-        assert n > 0
-        stream = np.ascontiguousarray(buf[:n])
+        yield "meshlet_%d" % case, np.ascontiguousarray(refs), np.ascontiguousarray(tris), style
+
+
+def encode_meshlet(ref, refs, tris):
+    buf = np.zeros(ref.meshopt_encodeMeshletBound(256, 256), np.uint8)
+    n = ref.meshopt_encodeMeshlet(_p(buf), len(buf), _p(refs), len(refs), _p(tris), len(tris))
+    assert n > 0
+    return np.ascontiguousarray(buf[:n])
+
+
+def test_meshlet_codec_against_reference(ref, stored):
+    ours = load_library()
+    cases = 0
+    for key, refs, tris, style in meshlet_cases():
+        vc, tc = len(refs), len(tris)
+        stream = _stream(ref, stored, key, lambda: encode_meshlet(ref, refs, tris))
+        if stream is None:
+            continue
+        n = len(stream)
         for ref_size in ((2, 4) if int(refs.max()) < (1 << 16) else (4,)):
-            want_r = np.zeros(vc + 2, np.uint16 if ref_size == 2 else np.uint32)
-            want_t = np.zeros((tc + 2) * 3 + 4, np.uint8)
-            assert ref.meshopt_decodeMeshlet(_p(want_r), vc, ref_size, _p(want_t), tc, 3, _p(stream), n) == 0
-            got_r = np.full(vc + 2, 0xEE, want_r.dtype)
+            got_r = np.full(vc + 2, 0xEE, np.uint16 if ref_size == 2 else np.uint32)
             got_t = np.full((tc + 2) * 3 + 4, 0xEE, np.uint8)
             assert ours.nvc_decode_meshlet_stream(_p(got_r), vc, ref_size, _p(got_t), tc, _p(stream), n) == 0, (vc, tc, style)
-            assert np.array_equal(got_r[:vc], want_r[:vc]) and np.array_equal(got_r[:vc].astype(np.uint32), refs.astype(want_r.dtype).astype(np.uint32))
-            assert np.array_equal(got_t[: tc * 3], want_t[: tc * 3]), (vc, tc, style)
+            if ref is not None:
+                want_r = np.zeros(vc + 2, got_r.dtype)
+                want_t = np.zeros((tc + 2) * 3 + 4, np.uint8)
+                assert ref.meshopt_decodeMeshlet(_p(want_r), vc, ref_size, _p(want_t), tc, 3, _p(stream), n) == 0
+                assert np.array_equal(got_r[:vc], want_r[:vc])
+                assert np.array_equal(got_t[: tc * 3], want_t[: tc * 3]), (vc, tc, style)
+            if key in stored:
+                reference_pins.check("%s ref_size %d" % (key, ref_size), *((want_r[:vc], want_t[: tc * 3]) if ref is not None else (got_r[:vc], got_t[: tc * 3])))
+            assert np.array_equal(got_r[:vc].astype(np.uint32), refs.astype(got_r.dtype).astype(np.uint32))
             assert (got_t[tc * 3 :] == 0xEE).all() and (got_r[vc:] == 0xEE).all()  # nothing written past the outputs
             a, b = tris.reshape(-1, 3), got_t[: tc * 3].reshape(-1, 3)
             assert ((a == b).all(1) | (np.roll(a, 1, 1) == b).all(1) | (np.roll(a, 2, 1) == b).all(1)).all()
             cases += 1
         # (a meshlet block carries no length of its own — it is parsed from its end — so a truncated block may still be a valid one)
         assert ours.nvc_decode_meshlet_stream(_p(got_r), vc, 4 if got_r.dtype == np.uint32 else 2, _p(got_t), tc, _p(stream), n - 1) in (0, -7)
-    assert cases >= 600
+    assert cases >= (600 if ref is not None else 100)

@@ -113,28 +113,35 @@ def test_kitten_cache_against_reference_geometry_and_digest():
     assert hashlib.sha256((md.view(np.uint8) * mask).tobytes()).hexdigest() == want["meshletdata_sha256_masked"]
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="needs the reference checkout to run its cache writer / loader")
-def test_fresh_reference_output_full_compare(tmp_path):
-    """Where the reference is present: run its writer + loader now and compare the whole decoded meshletdata of kitten."""
-    subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref"], check=True)
-    subprocess.run([os.path.join(ROOT, "oracle", "_ref", "write_cache"), str(tmp_path / "kitten"), "/root/reference/data/kitten.obj"], check=True, stdout=subprocess.DEVNULL)
-    assert open(tmp_path / "kitten.z.cache", "rb").read() == open(os.path.join(GOLDEN, "kitten.z.cache"), "rb").read()
-    c = scene_cache.SceneCache(str(tmp_path / "kitten.z.cache"))
-    ref = np.fromfile(tmp_path / "kitten.z.meshletdata", dtype="<u4")
-    mask = meaningful_bytes(c.section("meshlets"), len(ref))
-    assert np.array_equal(c.section("meshletdata").view(np.uint8) * mask, ref.view(np.uint8) * mask)
-    r = scene_cache.SceneCache(str(tmp_path / "kitten.raw.cache"))
-    assert np.array_equal(r.section("meshlets"), c.section("meshlets")) and len(r.section("indices")) == r.header.indexCount
-    assert np.array_equal(c.section("vertices"), r.section("vertices"))
-    assert np.array_equal(c.section("indices"), np.fromfile(tmp_path / "kitten.z.indices", dtype="<u4"))
-    # a glTF scene with several meshes and materials as well
-    subprocess.run([os.path.join(ROOT, "oracle", "_ref", "write_cache"), str(tmp_path / "pirate"), "/root/reference/extern/meshoptimizer/demo/pirate.glb"], check=True, stdout=subprocess.DEVNULL)
-    pz, pr = scene_cache.SceneCache(str(tmp_path / "pirate.z.cache")), scene_cache.SceneCache(str(tmp_path / "pirate.raw.cache"))
-    assert np.array_equal(pz.section("vertices"), pr.section("vertices"))
-    assert np.array_equal(pz.section("indices"), np.fromfile(tmp_path / "pirate.z.indices", dtype="<u4"))
-    ref = np.fromfile(tmp_path / "pirate.z.meshletdata", dtype="<u4")
-    mask = meaningful_bytes(pz.section("meshlets"), len(ref))
-    assert np.array_equal(pz.section("meshletdata").view(np.uint8) * mask, ref.view(np.uint8) * mask)
+def test_fresh_reference_output_full_compare(tmp_path, request):
+    """kitten.obj and pirate.glb (the glTF importer: several meshes and materials) through the reference's writer + loader:
+    where the reference is present it runs now and its compressed caches must equal the stored ones; every section the
+    product's decoders read from those caches equals what the reference's loader decodes (meshletdata, padding bytes
+    masked; indices) and what its uncompressed cache holds (Meshlet[], vertices).  Elsewhere the reference's sections are
+    the pinned ones (reference_pins)."""
+    import reference_pins
+    from refshader_lib import REFERENCE
+
+    live = os.path.isdir(os.path.join(REFERENCE, "src"))
+    if live:
+        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref", "REF=" + REFERENCE], check=True)
+    with reference_pins.pinned(request, live):
+        for name, model, stored in (("kitten", "data/kitten.obj", "kitten.z.cache"), ("pirate_glb", "extern/meshoptimizer/demo/pirate.glb", "pirate_glb.z.cache")):
+            c = scene_cache.SceneCache(os.path.join(GOLDEN, stored))
+            md = c.section("meshletdata")
+            ours = {"meshletdata": md.view(np.uint8) * meaningful_bytes(c.section("meshlets"), len(md)), "meshlets": c.section("meshlets"), "vertices": c.section("vertices"), "indices": c.section("indices").astype("<u4")}
+            if live:
+                prefix = str(tmp_path / name)
+                subprocess.run([os.path.join(ROOT, "oracle", "_ref", "write_cache"), prefix, os.path.join(REFERENCE, model)], check=True, stdout=subprocess.DEVNULL)
+                assert open(prefix + ".z.cache", "rb").read() == open(os.path.join(GOLDEN, stored), "rb").read(), name
+                ref = np.fromfile(prefix + ".z.meshletdata", dtype="<u4")
+                r = scene_cache.SceneCache(prefix + ".raw.cache")
+                assert len(r.section("indices")) == r.header.indexCount
+                want = {"meshletdata": ref.view(np.uint8) * meaningful_bytes(c.section("meshlets"), len(ref)), "meshlets": r.section("meshlets"), "vertices": r.section("vertices"), "indices": np.fromfile(prefix + ".z.indices", dtype="<u4")}
+                for k in ours:
+                    assert np.array_equal(ours[k], want[k]), (name, k)
+            for k in ours:
+                reference_pins.check("%s %s" % (name, k), want[k] if live else ours[k])
 
 
 def test_corrupt_and_truncated_files_are_rejected(tmp_path):
@@ -308,15 +315,33 @@ def test_decoders_under_address_and_ub_sanitizers(tmp_path):
         assert "mutations 1500" in run.stdout
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src") and not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "libanim_ref.so")), reason="needs glm from the reference (oracle/_ref/libanim_ref.so)")
-def test_animation_blend_against_glm_on_random_keyframes():
+def load_glm():
+    """oracle/_ref/libanim_ref.so (glm of the reference, see oracle/refscene/anim_ref.cpp), or None where it is neither built
+    nor buildable"""
+    from refshader_lib import REFERENCE
+
+    if os.path.isdir(os.path.join(REFERENCE, "src")):
+        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref", "REF=" + REFERENCE], check=True)
+    so = os.path.join(ROOT, "oracle", "_ref", "libanim_ref.so")
+    return ctypes.CDLL(so) if os.path.exists(so) else None
+
+
+def test_animation_blend_against_glm_on_random_keyframes(request):
     """Property test of nvc_host_animate's blend against glm::mix / glm::slerp themselves (oracle/refscene/anim_ref.cpp):
     random unit and non-unit quaternions, nearly identical ones (glm's lerp shortcut), opposite ones (sign flip), exact 0 / 1
-    and tiny blend factors — bit for bit."""
-    if os.path.isdir("/root/reference/src"):
-        subprocess.run(["make", "-s", "-C", os.path.join(ROOT, "oracle"), "ref"], check=True)
-    glm = ctypes.CDLL(os.path.join(ROOT, "oracle", "_ref", "libanim_ref.so"))
-    glm.anim_ref_blend.argtypes = [ctypes.c_void_p, ctypes.c_float, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_float, ctypes.c_void_p, ctypes.c_float, ctypes.c_void_p]
+    and tiny blend factors — bit for bit.  Without glm its results are the pinned ones (reference_pins), one pin per factor."""
+    import reference_pins
+
+    glm = load_glm()
+    with reference_pins.pinned(request, glm is not None):
+        _animation_blend(glm)
+
+
+def _animation_blend(glm):
+    import reference_pins
+
+    if glm is not None:
+        glm.anim_ref_blend.argtypes = [ctypes.c_void_p, ctypes.c_float, ctypes.c_void_p, ctypes.c_void_p, ctypes.c_float, ctypes.c_void_p, ctypes.c_float, ctypes.c_void_p]
     rng = np.random.default_rng(8)
     n = 4000
     keys = np.zeros(2 * n, dtype=layout.KEYFRAME_DTYPE)
@@ -342,9 +367,15 @@ def test_animation_blend_against_glm_on_random_keyframes():
         idx, val = host.animate(anims, keys, t, draws)  # index = t in [0, 1): keyframe 0 -> 1, blend factor float(t)
         assert len(idx) == n
         a = np.float32(t - np.floor(t))
+        got = np.concatenate([draws["position"], draws["scale"][:, None], draws["orientation"]], 1).astype(np.float32)
+        if glm is None:
+            reference_pins.check("t = %r" % t, got)
+            continue
+        want = np.zeros_like(got)
         for i in range(0, n, 1):
             k0, k1 = keys[2 * i], keys[2 * i + 1]
             glm.anim_ref_blend(k0["translation"].ctypes.data, float(k0["scale"]), k0["rotation"].ctypes.data, k1["translation"].ctypes.data, float(k1["scale"]), k1["rotation"].ctypes.data, float(a), out.ctypes.data)
-            got = np.concatenate([draws["position"][i], [draws["scale"][i]], draws["orientation"][i]]).astype(np.float32)
-            same = (got.view(np.uint32) == out.view(np.uint32)) | (np.isnan(got) & np.isnan(out))
-            assert same.all(), (t, i, got, out)
+            want[i] = out
+            same = (got[i].view(np.uint32) == out.view(np.uint32)) | (np.isnan(got[i]) & np.isnan(out))
+            assert same.all(), (t, i, got[i], out)
+        reference_pins.check("t = %r" % t, want)
